@@ -1,6 +1,6 @@
 """bench.py — graphs/sec through GPSLayer forward+backward on PCQM4M-shaped synthetic batches.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* is one GPSLayer forward+backward (training mode, BatchNorm batch statistics, dropout as
@@ -15,6 +15,10 @@ inside the step.  One JSON line is printed by rank 0.
   roofline  dominant kernel of the step, timed live with CUDA events around its C-ABI stage call
   cpu_baseline  the reference's own GPSLayer (oracle/_ref run verbatim under oracle/ref_shim.py; the
             oracle port if the files are absent) on the host cores, bounded sample of the same workload
+
+--dump-outputs DIR writes what the last timed step returned to its caller (x_out, edge_out, grad_x, grad_edge_attr,
+grad.<parameter>) as float32 DIR/<name>.npy.  Inputs, weights and dropout streams are seeded, so two builds run with
+the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -45,6 +49,7 @@ WORKLOADS = {
 }
 NUM_BATCHES = 8          # rotating distinct batches
 L2_FLUSH_BYTES = 256 << 20
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks():
@@ -246,6 +251,28 @@ def workload_config(name, spec, local, glob, heads, drop, adrop, n_gpus):
 
 
 # ================================================================================ our arm
+def dump_outputs(path, out, x_in, e_in, layer, gated):
+    """Writes one step's layer outputs, input gradients and parameter gradients as float32 .npy files; beyond
+    DUMP_LIMIT_BYTES in all, every array keeps the same share of its rows, chosen with a fixed seed."""
+    import numpy as np
+    arrays = {"x_out": out.x, "grad_x": x_in.grad}
+    if gated:
+        arrays["edge_out"] = out.edge_attr
+    if e_in.grad is not None:
+        arrays["grad_edge_attr"] = e_in.grad
+    arrays.update({"grad." + n: p.grad for n, p in layer.named_parameters() if p.grad is not None})
+    arrays = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(v.numel() * 4 for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        gen = torch.Generator().manual_seed(0)
+        for k, v in arrays.items():
+            keep = max(1, v.shape[0] * DUMP_LIMIT_BYTES // total)
+            arrays[k] = v[torch.randperm(v.shape[0], generator=gen)[:keep].sort().values]
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v.numpy())
+
+
 def trace(msg):
     """GPS_BENCH_TRACE=1: stage markers on stderr (+ a watchdog that dumps every thread's stack if a stage hangs)."""
     if os.environ.get("GPS_BENCH_TRACE") == "1":
@@ -322,7 +349,7 @@ def run_ours(args):
             torch.autograd.backward([out.x], [ctx])
         if reduce:
             allreduce_grads()
-        return out, x_in
+        return out, x_in, bb.edge_attr
 
     def barrier():
         if world > 1:
@@ -339,20 +366,21 @@ def run_ours(args):
     trace("capture")
     graphs = None
     graphs_local = None            # the same step without the collectives (N > 1: exposes the all-reduce cost)
+    results = None                 # per graph: the (out, x_in, e_in) its replays overwrite
     launches_per_step = None
     collective_in_graph = False
 
     def capture_all(reduce):
-        out = []
+        out, res = [], []
         nonlocal launches_per_step
         for i in range(NUM_BATCHES):
             g = torch.cuda.CUDAGraph()
             l0 = lib.gps_launch_count()
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                step(i, reduce=reduce)
+                res.append(step(i, reduce=reduce))
             launches_per_step = lib.gps_launch_count() - l0
             out.append(g)
-        return out
+        return out, res
 
     if args.graph:
         side = torch.cuda.Stream()
@@ -364,7 +392,7 @@ def run_ours(args):
         barrier()
         if world > 1 and os.environ.get("GPS_BENCH_NCCL_IN_GRAPH") == "1":
             try:     # NCCL collectives captured in the same graph as the step (measured: ~0.5 ms of host time per launch)
-                graphs = capture_all(True)
+                graphs, results = capture_all(True)
                 collective_in_graph = True
             except Exception as e:   # noqa: BLE001
                 sys.stderr.write(f"[bench] capturing the collectives failed ({e!r}); they run after each replay\n")
@@ -372,17 +400,17 @@ def run_ours(args):
                 torch.cuda.synchronize()
         # default: the graph holds fwd+bwd and records the gradient-group events as external event nodes; the
         # collectives are enqueued after each replay and wait on those events (overlap without NCCL graph nodes)
-        graphs_local = capture_all(False)
+        graphs_local, results_local = capture_all(False)
         if graphs is None:
-            graphs = graphs_local
+            graphs, results = graphs_local, results_local
 
     def run_step(i):
         if graphs is None:
-            step(i)
-        else:
-            graphs[i % NUM_BATCHES].replay()
-            if world > 1 and not collective_in_graph:
-                allreduce_grads()
+            return step(i)
+        graphs[i % NUM_BATCHES].replay()
+        if world > 1 and not collective_in_graph:
+            allreduce_grads()
+        return results[i % NUM_BATCHES]
 
     trace("graph warm-up")
     for i in range(args.warmup):
@@ -399,7 +427,7 @@ def run_ours(args):
         flush.zero_()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        run_step(i)
+        last = run_step(i)
         e1.record()
         evs.append((e0, e1))
     host_ms = (time.perf_counter() - host_t0) * 1e3 / args.steps   # host enqueue time per step (no sync inside)
@@ -411,6 +439,8 @@ def run_ours(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last, layer, gated)
 
     # N > 1: the same replays without the collectives -> what the all-reduce still costs after overlap
     trace("no-collective replays")
@@ -726,7 +756,12 @@ def main():
     ap.add_argument("--workload", default="pcqm4m-small", choices=sorted(WORKLOADS))
     ap.add_argument("--precision", default="fp32", choices=["fp32", "bf16"])
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="time eager launches instead of CUDA-graph replays")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs and gradients as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,9 +6,10 @@ does; it fails loudly when its CUDA library is missing.
 
 PARITY PINNING.  The reference's own tests hold *no* golden vectors for this path (SURVEY.md
 section 4 / 8c: "parity unpinned" by the reference).  This restatement is therefore pinned against
-outputs of the reference itself run here: ``tests/test_oracle.py::test_oracle_equals_reference_live``
-executes the reference's own layer files verbatim (oracle/ref_shim.py) and asserts equality with this
-file in fp64 (<=1e-10 outputs, <=1e-9 gradients), forward and backward, for seven variants;
+outputs of the reference itself: ``tests/test_oracle.py::test_oracle_equals_reference_live`` asserts
+equality of this file in fp64 with the reference's own layer files run verbatim (oracle/ref_shim.py) by
+tests/golden/make_golden.py, kept in tests/golden/reference/ as seeded samples and full-tensor sums
+(<=1e-10 outputs, <=1e-9 gradients), forward and backward, for seven variants;
 ``test_oracle_matches_golden_fp64`` / ``test_oracle_fp32_close_to_golden`` pin it to the fixtures (2e-6 / 5e-4); and
 ``tests/golden/*.pt`` (made by tests/golden/make_golden.py from the reference-verbatim layer in
 fp64) travel to the GPU box.  The published parameter totals (README.md:77-79 of the reference)

@@ -13,7 +13,8 @@ from graphgps_b200 import _lib
 from graphgps_b200.batch import batch_from_lists, make_batch
 from graphgps_b200.graph import GraphStructure, graph_of
 from oracle.gps_oracle import OracleGPSLayer
-from util import compare, golden_batch, golden_names, load_golden, rel_err, rel_l2, run_layer
+from util import (check_summary, compare, golden_batch, golden_names, load_golden, load_reference_golden, rel_err,
+                  rel_l2, run_layer)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -556,17 +557,12 @@ def _inject_gatedgcn_dropout(local, mx, me):
 
 def test_three_layer_stack_matches_reference_stack():
     """GPSModel chains L GPSLayers, each consuming the previous layer's batch.x AND batch.edge_attr
-    (graphgps/network/gps_model.py:100,105-108).  Three CUDA layers chained vs three reference-verbatim layers
-    (oracle/_ref under the shim; the oracle restatement when the reference files are absent), fp64 target:
-    outputs, input gradients and every layer's parameter gradients."""
-    from oracle.ref_shim import find_reference_layer_dir, load_reference
+    (graphgps/network/gps_model.py:100,105-108).  Three CUDA layers chained vs three oracle layers in fp64, whose
+    results are pinned to those of three chained reference-verbatim layers (tests/golden/reference/stack3.pt, from
+    make_golden.py): outputs, input gradients and every layer's parameter gradients."""
     d, heads, L = 64, 4, 3
     torch.manual_seed(11)
-    if find_reference_layer_dir() is not None:
-        mk = lambda: load_reference().GPSLayer(d, "CustomGatedGCN", "Transformer", heads)   # noqa: E731
-    else:
-        mk = lambda: OracleGPSLayer(d, "CustomGatedGCN", "Transformer", heads)              # noqa: E731
-    refs = [mk() for _ in range(L)]
+    refs = [OracleGPSLayer(d, "CustomGatedGCN", "Transformer", heads) for _ in range(L)]
     ours = []
     for r in refs:
         m = graphgps_b200.GPSLayer(d, "CustomGatedGCN", "Transformer", heads)
@@ -575,6 +571,11 @@ def test_three_layer_stack_matches_reference_stack():
     b = make_batch("zinc-gatedgcn", seed=13, dim=d, num_graphs=24)
     g = torch.Generator().manual_seed(6)
     ct_x, ct_e = torch.randn(b.x.shape, generator=g), torch.randn(b.edge_attr.shape, generator=g)
+    fix = load_reference_golden("stack3")
+    check_summary({f"{li}.{k}": v for li, r in enumerate(refs) for k, v in r.state_dict().items()}, fix["state"], 1e-12,
+                  "seeded weights differ from make_golden.py's", scaled=True)
+    check_summary({"x": b.x, "edge_attr": b.edge_attr, "edge_index": b.edge_index, "batch": b.batch, "ct_x": ct_x,
+                   "ct_e": ct_e}, fix["inputs"], 1e-12, "seeded batch differs from make_golden.py's", scaled=True)
 
     def run(layers, bb, dev, dt):
         bb.x.requires_grad_(True)
@@ -588,6 +589,10 @@ def test_three_layer_stack_matches_reference_stack():
 
     rb = _to(b.clone(), "cpu", torch.float64)
     r = run([m.double() for m in refs], rb, "cpu", torch.float64)
+    check_summary({"x": r[0], "e": r[1], "gx": r[2], "ge": r[3]}, fix["outputs"], 1e-9, "fp64 target vs reference",
+                  scaled=True)
+    check_summary({f"{li}.{n}": t for li in range(L) for n, t in r[4][li].items()}, fix["grads"], 1e-9,
+                  "fp64 target vs reference parameter gradients", scaled=True)
     o = run(ours, b.clone().to(DEV), DEV, torch.float32)
     for name, a, t in (("x", o[0], r[0]), ("e", o[1], r[1])):
         assert rel_err(a, t) < 1e-3, (name, rel_err(a, t))

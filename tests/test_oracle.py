@@ -1,13 +1,12 @@
 """CPU: pins the oracle (oracle/gps_oracle.py) against the committed golden fixtures (outputs of the
-reference's own layer files, fp64) and, when the reference files are present, against the reference
-run live under oracle/ref_shim.py.  Also the published parameter-count KATs (README.md:77-79)."""
+reference's own layer files, fp64, run under oracle/ref_shim.py by tests/golden/make_golden.py).  Also the
+published parameter-count KATs (README.md:77-79)."""
 import pytest
 import torch
 
 from oracle.gps_oracle import OracleGPSLayer, param_count
-from oracle.ref_shim import find_reference_layer_dir, load_reference
 from graphgps_b200.batch import make_batch
-from util import compare, golden_batch, golden_names, load_golden, run_layer
+from util import check_summary, compare, golden_batch, golden_names, load_golden, load_reference_golden, run_layer
 
 
 @pytest.mark.parametrize("name", golden_names())
@@ -32,31 +31,28 @@ def test_oracle_fp32_close_to_golden(name):
     compare(res, fix, 5e-4, f"oracle fp32 vs golden {name}")
 
 
-@pytest.mark.skipif(find_reference_layer_dir() is None, reason="reference layer files not present")
 @pytest.mark.parametrize("local,glob", [("CustomGatedGCN", "Transformer"), ("GINE", "Transformer"),
                                         ("CustomGatedGCN", "Performer"), ("None", "Transformer"),
                                         ("GINE", "None"), ("GCN", "Transformer"), ("GCN", "None")])
 def test_oracle_equals_reference_live(local, glob):
-    ref = load_reference()
+    """The oracle in fp64 against the reference's own layer files run in fp64 on the same seeded weights and batch
+    (tests/golden/reference/oracle_live.pt, written by make_golden.py): outputs to 1e-10, gradients to 1e-9."""
+    fix = load_reference_golden("oracle_live")[f"{local}-{glob}"]
     torch.manual_seed(3)
-    R = ref.GPSLayer(32, local, glob, 4).double()
     O = OracleGPSLayer(32, local, glob, 4).double()
-    O.load_state_dict(R.state_dict(), strict=True)
     b = make_batch("zinc-gatedgcn", seed=5, dim=32, num_graphs=7, dtype=torch.float64)
-    b1, b2 = b.clone(), b.clone()
-    for bb in (b1, b2):
-        bb.x.requires_grad_(True)
-        bb.edge_attr.requires_grad_(True)
-    x1, x2 = b1.x, b2.x
-    o1, o2 = R(b1), O(b2)
-    (o1.x ** 2).sum().backward()
-    (o2.x ** 2).sum().backward()
-    assert (o1.x - o2.x).abs().max() < 1e-10
-    assert (x1.grad - x2.grad).abs().max() < 1e-9
-    po = dict(O.named_parameters())
-    for n, p in R.named_parameters():
-        if p.grad is not None:
-            assert (p.grad - po[n].grad).abs().max() < 1e-9, n
+    check_summary(O.state_dict(), fix["state"], 1e-12, "seeded weights differ from make_golden.py's", scaled=True)
+    check_summary({"x": b.x, "edge_attr": b.edge_attr, "edge_index": b.edge_index, "batch": b.batch}, fix["inputs"],
+                  1e-12, "seeded batch differs from make_golden.py's", scaled=True)
+    b.x.requires_grad_(True)
+    b.edge_attr.requires_grad_(True)
+    x_in = b.x
+    o = O(b)
+    (o.x ** 2).sum().backward()
+    check_summary({"x": o.x}, fix["outputs"], 1e-10, "oracle vs reference outputs")
+    check_summary({"grad_x": x_in.grad}, fix["grad_x"], 1e-9, "oracle vs reference input gradient")
+    check_summary({n: p.grad for n, p in O.named_parameters() if p.grad is not None}, fix["grads"], 1e-9,
+                  "oracle vs reference parameter gradients")
 
 
 def test_gcn_restatements_agree_with_self_loops_and_isolated_nodes():

@@ -47,6 +47,51 @@ def run_layer(layer, batch, fix, backward=True):
     return res
 
 
+def load_reference_golden(name):
+    """tests/golden/reference/<name>.pt: sampled outputs of the reference's own layer files (make_golden.py)."""
+    return torch.load(os.path.join(GOLDEN_DIR, "reference", name + ".pt"), weights_only=False)
+
+
+def sample_summary(tensors, k, seed=0):
+    """What a reference golden keeps of each named tensor, in fp64: k entries at fixed, seeded positions (all of a
+    smaller tensor) and the full tensor's sum, sum of magnitudes and largest magnitude."""
+    g = torch.Generator().manual_seed(seed)
+    names, count, numel, idx, val, stats = [], [], [], [], [], []
+    for n, t in tensors.items():
+        f = t.detach().cpu().double().flatten()
+        i = torch.randperm(f.numel(), generator=g)[:k]
+        names.append(n)
+        count.append(i.numel())
+        numel.append(f.numel())
+        idx.append(i.int())
+        val.append(f[i])
+        stats.append(torch.stack([f.sum(), f.abs().sum(), f.abs().max()]))
+    return {"names": names, "count": count, "numel": numel, "idx": torch.cat(idx), "val": torch.cat(val),
+            "stats": torch.stack(stats)}
+
+
+def check_summary(tensors, summ, tol, what, scaled=False):
+    """Asserts what max|a - b| <= tol * s implies for every tensor of a sample_summary: each stored entry within
+    tol * s, the sum, the sum of magnitudes within numel * tol * s, and the largest magnitude within tol * s.
+    s = 1, or max(1, max|b|) when scaled."""
+    assert sorted(tensors) == sorted(summ["names"]), (what, sorted(set(tensors) ^ set(summ["names"])))
+    bad, off = {}, 0
+    for n, c, ne, st in zip(summ["names"], summ["count"], summ["numel"], summ["stats"]):
+        f = tensors[n].detach().cpu().double().flatten()
+        i, v = summ["idx"][off:off + c].long(), summ["val"][off:off + c]
+        off += c
+        if f.numel() != ne:
+            bad[n] = ("numel", f.numel(), ne)
+            continue
+        s = max(1.0, float(st[2])) if scaled else 1.0
+        got = torch.stack([f.sum(), f.abs().sum(), f.abs().max()])
+        err = max(float((f[i] - v).abs().max()) / s, float((got[:2] - st[:2]).abs().max()) / (ne * s),
+                  float((got[2] - st[2]).abs()) / s)
+        if not err <= tol:
+            bad[n] = err
+    assert not bad, f"{what}: tolerance {tol} exceeded: {bad}"
+
+
 def rel_err(a, b):
     """max |a-b| / max(1, max|b|): absolute on O(1) (BatchNorm-normalised) data, relative on large."""
     a, b = a.double(), b.double()

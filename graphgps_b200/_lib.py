@@ -69,7 +69,10 @@ class GpsLayerArgs(C.Structure):
         ("x_planes_in", GpsPlanes), ("e_planes_in", GpsPlanes), ("x_planes_out", GpsPlanes), ("e_planes_out", GpsPlanes),
         ("wplanes", _fp), ("wplanes_bytes", C.c_int64), ("wplanes_valid", C.c_int32), ("reserved2", C.c_int32),
         ("ev_grads_mid", _fp), ("ev_grads_done", _fp),
+        ("pe", _fp), ("pe_dim", C.c_int64), ("grad_pe", _fp), ("es_r0", GpsLinear), ("es_r1", GpsLinear),
     ]
+
+ES_FLAG = 1   # GpsLayerArgs.reserved1 bit 0: EquivStableLapPE edge gate
 
 
 class GpsLayerPlan(C.Structure):
@@ -93,6 +96,12 @@ SYMBOLS = {
     "gps_gemm": (C.c_int, [_fp, _i64, _i32, _fp, _i64, _i32, _fp, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _fp]),
     "gps_gatedgcn_aggregate_forward": (C.c_int, [C.POINTER(GpsGraph), _i64, _fp, _fp, _fp, _fp, _i64, _fp, _fp,
                                                  _fp, _fp, _fp]),
+    "gps_es_gate_forward": (C.c_int, [C.POINTER(GpsGraph), _fp, _i64, _i64, _i32] + [_fp] * 6 + [_fp]),
+    "gps_gatedgcn_es_aggregate_forward": (C.c_int, [C.POINTER(GpsGraph), _i64, _fp, _fp, _fp, _fp, _i64, _fp, _fp,
+                                                    _fp, _fp, _fp, _fp]),
+    "gps_es_gate_backward_workspace_bytes": (_i64, [_i64, _i64]),
+    "gps_es_gate_backward": (C.c_int, [_i64, _i64, _i32] + [_fp] * 12 + [_fp, _i64, _fp]),
+    "gps_es_pe_backward": (C.c_int, [C.POINTER(GpsGraph), _fp, _i64, _fp, _fp, _fp]),
     "gps_gine_aggregate_forward": (C.c_int, [C.POINTER(GpsGraph), _i64, _fp, _fp, _f32, _fp, _fp]),
     "gps_attention_forward": (C.c_int, [C.POINTER(GpsGraph), _i64, _i64, _fp, _fp, _fp, _i64, _fp, _i64, _fp,
                                         _f32, _u64, _u64, _fp]),

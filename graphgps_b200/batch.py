@@ -200,3 +200,28 @@ def batch_from_lists(sizes, edge_lists, d, seed=0) -> GraphBatch:
     batch = torch.repeat_interleave(torch.arange(B, dtype=torch.int64), sizes_t)
     return GraphBatch(x=x, edge_index=edge_index, edge_attr=edge_attr, batch=batch,
                       num_graphs=B, ptr=ptr)
+
+
+def add_equivstable_pe(batch: GraphBatch, dim: Optional[int] = None, seed: int = 0, max_freqs: int = 8,
+                       scale: float = 1.0) -> GraphBatch:
+    """Attaches an encoder-like ``pe_EquivStableLapPE`` [N, dim] (default dim = batch.x's width) to ``batch``.
+
+    Stands in for the EquivStableLapPE encoder's output (graphgps/encoder/equivstable_laplace_pos_encoder.py:46-49:
+    Linear(max_freqs -> dim) over the Laplacian eigenvectors): per-graph L2-normalised random "eigenvector" columns
+    [N, max_freqs] through a seeded Linear(max_freqs, dim) with torch's default init, times ``scale``.  Full scale with
+    default mlp_r_ij weights saturates most edge gates near 1; scale 0.3 keeps them spread.  Uses its own generator, so
+    the batch's other tensors (and ``make_batch``'s stream) are untouched."""
+    d = int(batch.x.shape[1]) if dim is None else dim
+    gen = torch.Generator().manual_seed(seed)
+    N = batch.num_nodes
+    ev = torch.randn(N, max_freqs, generator=gen)
+    gid = batch.batch.cpu()
+    B = int(batch.num_graphs) if batch.num_graphs is not None else (int(gid.max()) + 1 if N else 0)
+    norm = torch.zeros(B, max_freqs).index_add_(0, gid, ev * ev).sqrt().clamp_min(1e-12)
+    ev = ev / norm[gid]
+    bound = 1.0 / max_freqs ** 0.5                       # nn.Linear's default init range
+    w = (torch.rand(d, max_freqs, generator=gen) * 2 - 1) * bound
+    b = (torch.rand(d, generator=gen) * 2 - 1) * bound
+    pe = (ev @ w.t() + b) * scale
+    batch.pe_EquivStableLapPE = pe.to(device=batch.x.device, dtype=batch.x.dtype)
+    return batch

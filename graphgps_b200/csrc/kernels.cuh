@@ -69,18 +69,40 @@ int colsum(const float* a, int64_t lda, int64_t rows, int64_t d, float* out, cud
 int copy2d(const float* src, int64_t lds, float* dst, int64_t ldd, int64_t rows, int64_t d, cudaStream_t stream);
 
 // ---- sparse (message passing) stages -------------------------------------------------------
+// gate != nullptr: EquivStableLapPE-gated aggregation, sigma_ij = sigmoid(e_ij) * gate[eid] (gate from es_gate_fwd)
 int gatedgcn_fwd(const GpsGraph& g, int64_t d, const float* Ax, const float* Bx, const float* Dx,
                  const float* Ex, int64_t ldy, float* Ce, float* xt, double* stats_x, double* stats_e,
-                 cudaStream_t stream);
+                 cudaStream_t stream, const float* gate = nullptr);
 // dst-ordered backward pass: reads g_xt (ld ldg), ehat, Bx; g_e holds the BN_e-path gradient on entry
 // and the total gradient w.r.t. e_ij on exit; writes g_num [N,d] and g_Dx (ld ldg).
+// gate != nullptr: the gated pass; it also writes the per-warp shares of d loss / d gate[eid] to
+// g_gate [E, gatedgcn_es_nwarps(d)]
 int gatedgcn_bwd_dst(const GpsGraph& g, int64_t d, const float* g_xt, int64_t ldg, const float* ehat,
                      const float* Bx, int64_t ldy, float* g_e, float* g_num, float* g_Dx,
-                     cudaStream_t stream, Planes g_e_p = Planes(), Planes g_Dx_p = Planes());
-// src-ordered backward pass: g_Ex_j = sum g_e_k, g_Bx_j = sum g_num[dst(k)] * sigmoid(ehat_k)
+                     cudaStream_t stream, Planes g_e_p = Planes(), Planes g_Dx_p = Planes(),
+                     const float* gate = nullptr, float* g_gate = nullptr);
+int gatedgcn_es_nwarps(int64_t d);
+// src-ordered backward pass: g_Ex_j = sum g_e_k, g_Bx_j = sum g_num[dst(k)] * sigmoid(ehat_k) [* gate_k]
 int gatedgcn_bwd_src(const GpsGraph& g, int64_t d, const float* g_e, const float* ehat, const float* g_num,
                      float* g_Ex, float* g_Bx, int64_t ldg, cudaStream_t stream, Planes g_Ex_p = Planes(),
-                     Planes g_Bx_p = Planes());
+                     Planes g_Bx_p = Planes(), const float* gate = nullptr);
+
+// ---- EquivStableLapPE edge gate (eslappe.cu; gatedgcn_layer.py:29-35, 99-103)
+// r_e = sum_c (PE_dst - PE_src)_c^2 ;  gate_e = sigmoid(W2 act(W1 r_e + b1) + b2)   (W1 [d,1], W2 [1,d])
+struct EsMlp {
+  const float *w1, *b1, *w2, *b2;
+  float *gw1, *gb1, *gw2, *gb2;
+};
+int es_gate_fwd(const GpsGraph& g, const float* pe, int64_t k, int64_t d, int act, const EsMlp& m, float* r, float* gate,
+                cudaStream_t stream);
+// workspace of es_gate_bwd: per-block partial sums of the mlp_r_ij gradients
+int64_t es_gate_bwd_bytes(int64_t E, int64_t d);
+// g_gate [E, nshare]: shares of d loss / d gate_e (summed in order).  Writes g_r [E] and the four parameter gradients
+// (added to the buffers when accumulate), deterministic: per-block partials, then a fixed-order final sum.
+int es_gate_bwd(int64_t E, int64_t d, int act, const EsMlp& m, const float* r, const float* gate, const float* g_gate,
+                int nshare, float* g_r, void* work, int64_t work_bytes, bool accumulate, cudaStream_t stream);
+// grad_pe_n = sum_{e in dst(n)} 2 g_r_e (PE_n - PE_src(e)) + sum_{e in src(n)} 2 g_r_e (PE_n - PE_dst(e))
+int es_pe_bwd(const GpsGraph& g, const float* pe, int64_t k, const float* g_r, float* grad_pe, cudaStream_t stream);
 int gine_fwd(const GpsGraph& g, int64_t d, const float* x, const float* e, float eps, float* out,
              cudaStream_t stream, Planes outp = Planes());
 // g_e[k] = g_o[dst(k)] * [x_src + e_k > 0];  (dst ordered)

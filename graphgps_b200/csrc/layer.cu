@@ -209,6 +209,13 @@ struct Plan {
   float *Wcat, *bcat, *Y1, *ehat, *xt, *xloc, *O, *lse, *hA, *s, *hid, *hid_pre, *t, *bnbuf;
   float *agg, *h1, *h1_pre;
   float* dinv;   // GCN: deg^-1/2 per node
+  // EquivStableLapPE edge gate (GpsLayerArgs.reserved1 bit 0, GatedGCN only): saved r_e, gate_e; backward workspace
+  // d loss / d gate shares [E, es_nw], d loss / d r [E] and the per-block partials of the mlp_r_ij gradients
+  bool es;
+  int es_nw;
+  float *es_r, *es_g, *es_ggate, *es_gr;
+  void* es_work;
+  int64_t es_work_bytes;
   // pre-packed bf16 hi/lo weight planes for the forward GEMMs (bulk-TMA B operand)
   uint8_t *pk_cat, *pk_C, *pk_out, *pk_ff1, *pk_ff2, *pk_g0, *pk_g1;
   // the same weights as MN-major planes for the data-gradient GEMMs of the backward pass (training only)
@@ -268,6 +275,11 @@ static int make_plan(const GpsLayerArgs* a, Plan* P, bool bind) {
   P->gated = a->local_type == GPS_LOCAL_GATEDGCN;
   P->gine = a->local_type == GPS_LOCAL_GINE;
   P->gcn = a->local_type == GPS_LOCAL_GCN;
+  P->es = (a->reserved1 & 1) != 0;
+  GPS_REQUIRE(!P->es || P->gated, GPS_ERR_UNSUPPORTED,
+              "equivstable_pe (reserved1 bit 0) is built for the GatedGCN local model only (local_type %d)", a->local_type);
+  GPS_REQUIRE(!P->es || a->d <= 1023, GPS_ERR_UNSUPPORTED, "equivstable_pe supports dim_h <= 1023 (got %lld)",
+              (long long)a->d);
   GPS_REQUIRE(a->local_type == GPS_LOCAL_NONE || P->gated || P->gine || P->gcn, GPS_ERR_ARG, "unknown local_type %d",
               a->local_type);
   GPS_REQUIRE(a->global_type == GPS_GLOBAL_NONE || a->global_type == GPS_GLOBAL_TRANSFORMER ||
@@ -307,6 +319,10 @@ static int make_plan(const GpsLayerArgs* a, Plan* P, bool bind) {
   if (P->gated) {
     P->ehat = S.alloc<float>(E * d);
     P->xt = S.alloc<float>(N * d);
+    if (P->es) {
+      P->es_r = S.alloc<float>(E);
+      P->es_g = S.alloc<float>(E);
+    }
   }
   if (P->gine) {
     P->agg = S.alloc<float>(N * d);
@@ -471,6 +487,13 @@ static int make_plan(const GpsLayerArgs* a, Plan* P, bool bind) {
   if (P->gated) {
     P->g_e = Bk.alloc<float>(E * d);
     P->g_num = Bk.alloc<float>(N * d);
+    if (P->es) {
+      P->es_nw = gatedgcn_es_nwarps(d);
+      P->es_ggate = Bk.alloc<float>(E * P->es_nw);
+      P->es_gr = Bk.alloc<float>(E);
+      P->es_work_bytes = es_gate_bwd_bytes(E, d);
+      P->es_work = Bk.alloc<uint8_t>(P->es_work_bytes);
+    }
   }
   if (P->gine) {
     P->g_h1 = Bk.alloc<float>(N * d);
@@ -558,6 +581,11 @@ static int check_bn(const GpsBatchNorm& b, const char* name) {
   return GPS_OK;
 }
 
+static EsMlp es_mlp(const GpsLayerArgs* a) {
+  return EsMlp{a->es_r0.weight, a->es_r0.bias, a->es_r1.weight, a->es_r1.bias,
+               a->es_r0.grad_weight, a->es_r0.grad_bias, a->es_r1.grad_weight, a->es_r1.grad_bias};
+}
+
 static int check_params(const GpsLayerArgs* a, const Plan& P) {
   GPS_REQUIRE(a->x && (P.E == 0 || a->edge_attr || !(P.gated || P.gine)), GPS_ERR_ARG,
               "missing x / edge_attr");
@@ -569,6 +597,11 @@ static int check_params(const GpsLayerArgs* a, const Plan& P) {
     GPS_TRY(check_linear(a->gcn_E, "local_model.E", true));
     GPS_TRY(check_bn(a->bn_node_x, "local_model.bn_node_x"));
     GPS_TRY(check_bn(a->bn_edge_e, "local_model.bn_edge_e"));
+  }
+  if (P.es) {
+    GPS_REQUIRE(a->pe && a->pe_dim > 0, GPS_ERR_ARG, "equivstable_pe: missing pe_EquivStableLapPE (pe / pe_dim)");
+    GPS_TRY(check_linear(a->es_r0, "local_model.mlp_r_ij.0", true));
+    GPS_TRY(check_linear(a->es_r1, "local_model.mlp_r_ij.2", true));
   }
   if (P.gine) {
     GPS_TRY(check_linear(a->gine_lin0, "local_model.nn.0", true));
@@ -775,6 +808,8 @@ static int layer_forward(const GpsLayerArgs* a, cudaStream_t st) {
     set_bpk(g, P.pk_C, d, d, 0);
     g.Ap = P.e_p; g.Bp = P.C_p;
     GPS_TRY(gemm(g, s2));
+    // EquivStableLapPE gate: PE and mlp_r_ij only, next to the edge projection (joined before the aggregation)
+    if (P.es) GPS_TRY(es_gate_fwd(a->graph, a->pe, a->pe_dim, d, act, es_mlp(a), P.es_r, P.es_g, s2));
   }
 
   // ---- node projections: [Ax|Bx|Dx|Ex|Q|K|V] = x Wcat^T + bcat  (gatedgcn_layer.py:57-61, MHA in_proj)
@@ -817,7 +852,7 @@ static int layer_forward(const GpsLayerArgs* a, cudaStream_t st) {
   // ---- local model
   if (P.gated) {
     GPS_TRY(gatedgcn_fwd(a->graph, d, P.Y1, P.Y1 + d, P.Y1 + 2 * d, P.Y1 + 3 * d, P.Wy, P.ehat, P.xt,
-                         stats(BN_X), stats(BN_E), st));
+                         stats(BN_X), stats(BN_E), st, P.es ? P.es_g : nullptr));
     // x_loc = x + drop(act(BN(x~)));  e_out = e + drop(act(BN(e^)))   (gatedgcn_layer.py:72-83)
     GPS_TRY(bn_act_residual2(P.xt, a->x, P.xloc, N, bn_view_fwd(P, a, BN_X, a->bn_node_x, N), drop(GPS_SITE_GCN_X), stats(BN_L),
                              P.ehat, a->edge_attr, a->edge_out, E, bn_view_fwd(P, a, BN_E, a->bn_edge_e, E),
@@ -1248,12 +1283,17 @@ static int layer_backward(const GpsLayerArgs* a, cudaStream_t st) {
     if (se != st) GPS_TRY(sd->order(se, st));
     // message/aggregate backward (SURVEY Appendix C)
     GPS_TRY(gatedgcn_bwd_dst(a->graph, d, P.gY1, P.Wy, P.ehat, P.Y1 + d, P.Wy, P.g_e, P.g_num, P.gY1 + 2 * d, st, P.ge_p,
-                             P.gY1_p.cols(2 * d)));
+                             P.gY1_p.cols(2 * d), P.es ? P.es_g : nullptr, P.es_ggate));
     GPS_TRY(gatedgcn_bwd_src(a->graph, d, P.g_e, P.ehat, P.g_num, P.gY1 + 3 * d, P.gY1 + d, P.Wy, st, P.gY1_p.cols(3 * d),
-                             P.gY1_p.cols(d)));
+                             P.gY1_p.cols(d), P.es ? P.es_g : nullptr));
     // C: dC = g_e^T e ; g_edge_attr = grad_edge_out + g_e C
     GPS_TRY(wfork(st));
     GPS_TRY(linear_wgrad(P.g_e, d, a->edge_attr, d, E, d, d, a->gcn_C.grad_weight, a->gcn_C.grad_bias, prec, s2, P.ge_p, P.e_p));
+    if (P.es) {   // EquivStableLapPE gate: mlp_r_ij gradients (MID group, final before ev_grads_mid) and d loss / d PE
+      GPS_TRY(es_gate_bwd(E, d, act, es_mlp(a), P.es_r, P.es_g, P.es_ggate, P.es_nw, P.es_gr, P.es_work, P.es_work_bytes,
+                          g_grads_accumulate, s2));
+      if (a->grad_pe) GPS_TRY(es_pe_bwd(a->graph, a->pe, a->pe_dim, P.es_gr, a->grad_pe, s2));
+    }
     GPS_TRY(mid_done());
     if (a->grad_edge_attr && E > 0) {
       GemmParams g;
@@ -1514,6 +1554,39 @@ extern "C" int gps_gatedgcn_aggregate_forward(const GpsGraph* g, int64_t d, cons
                                               double* stats_x, double* stats_e, void* stream) {
   GPS_REQUIRE(g && Ax && Bx && Dx && Ex && (Ce || g->E == 0) && xt, GPS_ERR_ARG, "gatedgcn_aggregate: null argument");
   return gatedgcn_fwd(*g, d, Ax, Bx, Dx, Ex, ldy, Ce, xt, stats_x, stats_e, (cudaStream_t)stream);
+}
+
+extern "C" int gps_es_gate_forward(const GpsGraph* g, const float* pe, int64_t pe_dim, int64_t d, int32_t act,
+                                   const float* w0, const float* b0, const float* w2, const float* b2, float* r, float* gate,
+                                   void* stream) {
+  GPS_REQUIRE(g && (act == GPS_ACT_RELU || act == GPS_ACT_GELU), GPS_ERR_ARG, "es_gate_forward: bad argument");
+  EsMlp m{w0, b0, w2, b2, nullptr, nullptr, nullptr, nullptr};
+  return es_gate_fwd(*g, pe, pe_dim, d, act, m, r, gate, (cudaStream_t)stream);
+}
+
+extern "C" int gps_gatedgcn_es_aggregate_forward(const GpsGraph* g, int64_t d, const float* Ax, const float* Bx,
+                                                 const float* Dx, const float* Ex, int64_t ldy, float* Ce, float* xt,
+                                                 double* stats_x, double* stats_e, const float* gate, void* stream) {
+  GPS_REQUIRE(g && Ax && Bx && Dx && Ex && (Ce || g->E == 0) && xt && (gate || g->E == 0), GPS_ERR_ARG,
+              "gatedgcn_es_aggregate: null argument");
+  return gatedgcn_fwd(*g, d, Ax, Bx, Dx, Ex, ldy, Ce, xt, stats_x, stats_e, (cudaStream_t)stream, gate);
+}
+
+extern "C" int64_t gps_es_gate_backward_workspace_bytes(int64_t E, int64_t d) { return es_gate_bwd_bytes(E, d); }
+
+extern "C" int gps_es_gate_backward(int64_t E, int64_t d, int32_t act, const float* w0, const float* b0, const float* w2,
+                                    const float* b2, const float* r, const float* gate, const float* g_gate, float* g_r,
+                                    float* grad_w0, float* grad_b0, float* grad_w2, float* grad_b2, void* workspace,
+                                    int64_t workspace_bytes, void* stream) {
+  GPS_REQUIRE(act == GPS_ACT_RELU || act == GPS_ACT_GELU, GPS_ERR_ARG, "es_gate_backward: unknown activation %d", act);
+  EsMlp m{w0, b0, w2, b2, grad_w0, grad_b0, grad_w2, grad_b2};
+  return es_gate_bwd(E, d, act, m, r, gate, g_gate, 1, g_r, workspace, workspace_bytes, false, (cudaStream_t)stream);
+}
+
+extern "C" int gps_es_pe_backward(const GpsGraph* g, const float* pe, int64_t pe_dim, const float* g_r, float* grad_pe,
+                                  void* stream) {
+  GPS_REQUIRE(g, GPS_ERR_ARG, "es_pe_backward: null graph");
+  return es_pe_bwd(*g, pe, pe_dim, g_r, grad_pe, (cudaStream_t)stream);
 }
 
 extern "C" int gps_gine_aggregate_forward(const GpsGraph* g, int64_t d, const float* x, const float* e, float eps,

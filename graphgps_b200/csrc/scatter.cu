@@ -13,6 +13,8 @@
 // atomics on feature data, deterministic order (edge-id order inside a segment) — and the
 // BatchNorm column statistics of the two outputs are reduced thread -> CTA -> global doubles.
 // Backward maths: SURVEY.md Appendix C.
+#include <algorithm>
+
 #include "kernels.cuh"
 
 namespace gps {
@@ -75,11 +77,13 @@ __device__ __forceinline__ void block_stats(float4* acc, double* const* ptrs, fl
   }
 }
 
-template <bool STATS>
+// GATED: EquivStableLapPE edge gate (gatedgcn_layer.py:99-103), sigma_ij = sigmoid(e_ij) * gate[eid], one scalar per
+// edge from eslappe.cu; the edge output e_ij stays ungated
+template <bool STATS, bool GATED>
 __global__ void __launch_bounds__(1024) k_gatedgcn_fwd(GpsGraph g, int d, const float* __restrict__ Ax, const float* __restrict__ Bx,
                                const float* __restrict__ Dx, const float* __restrict__ Ex, int64_t ldy,
                                float* __restrict__ Ce, float* __restrict__ xt, double* stats_x,
-                               double* stats_e) {
+                               double* stats_e, const float* __restrict__ gate) {
   extern __shared__ float4 sm[];
   const int c = threadIdx.x * 4, ry = threadIdx.y, RY = blockDim.y;
   float4 acc[4] = {f4zero(), f4zero(), f4zero(), f4zero()};  // sum x~, sum x~^2, sum e, sum e^2
@@ -87,9 +91,11 @@ __global__ void __launch_bounds__(1024) k_gatedgcn_fwd(GpsGraph g, int d, const 
     const float4 dx = ld4(Dx + i * ldy + c);
     float4 num = f4zero(), den = f4zero();
     const int kb = g.dst_ptr[i], ke = g.dst_ptr[i + 1];
-    // two edges per iteration: 6 independent 128-bit gathers in flight per thread (the loop is latency bound)
-    for (int k = kb; k < ke; k += 2) {
-      const bool two = k + 1 < ke;
+    // two edges per iteration: 6 independent 128-bit gathers in flight per thread (the loop is latency bound).  The
+    // gated variant takes one: with the gate scalars the statistics instantiation would exceed 64 registers and spill.
+#pragma unroll 1
+    for (int k = kb; k < ke; k += GATED ? 1 : 2) {
+      const bool two = !GATED && k + 1 < ke;
       const int j0 = g.dst_src[k], j1 = two ? g.dst_src[k + 1] : j0;
       const int64_t e0 = g.dst_eid[k], e1 = two ? g.dst_eid[k + 1] : e0;
       const float4 ex0 = ld4(Ex + (int64_t)j0 * ldy + c), bx0 = ld4(Bx + (int64_t)j0 * ldy + c);
@@ -98,7 +104,8 @@ __global__ void __launch_bounds__(1024) k_gatedgcn_fwd(GpsGraph g, int d, const 
       float4 c1 = ld4(Ce + e1 * d + c);
       c0 = f4add(c0, f4add(dx, ex0));
       st4(Ce + e0 * d + c, c0);
-      const float4 s0 = sigmoid4(c0);
+      float4 s0 = sigmoid4(c0);
+      if (GATED) s0 = f4scale(s0, gate[e0]);
       num = f4fma(s0, bx0, num);
       den = f4add(den, s0);
       if (STATS) {
@@ -108,7 +115,8 @@ __global__ void __launch_bounds__(1024) k_gatedgcn_fwd(GpsGraph g, int d, const 
       if (two) {
         c1 = f4add(c1, f4add(dx, ex1));
         st4(Ce + e1 * d + c, c1);
-        const float4 s1 = sigmoid4(c1);
+        float4 s1 = sigmoid4(c1);
+        if (GATED) s1 = f4scale(s1, gate[e1]);
         num = f4fma(s1, bx1, num);
         den = f4add(den, s1);
         if (STATS) {
@@ -132,53 +140,77 @@ __global__ void __launch_bounds__(1024) k_gatedgcn_fwd(GpsGraph g, int d, const 
   }
 }
 
+// GATED: sigma = sigmoid(ehat) * gate[eid].  The row of a node is padded to whole warps (blockDim.x = round_up(d/4, 32),
+// lanes with c >= d only take part in the shuffles), and each warp writes its share of d loss / d gate[eid] =
+// sum_c gs_c sigmoid(ehat)_c to g_gate[eid * nwarps + warp]; es_gate_bwd sums the shares in a fixed order.
+template <bool GATED>
 __global__ void k_gatedgcn_bwd_dst(GpsGraph g, int d, const float* __restrict__ g_xt, int64_t ldg,
                                    const float* __restrict__ ehat, const float* __restrict__ Bx, int64_t ldy,
                                    float* __restrict__ g_e, float* __restrict__ g_num,
-                                   float* __restrict__ g_Dx, Planes g_e_p, Planes g_Dx_p) {
+                                   float* __restrict__ g_Dx, Planes g_e_p, Planes g_Dx_p,
+                                   const float* __restrict__ gate, float* __restrict__ g_gate) {
   const int c = threadIdx.x * 4, ry = threadIdx.y, RY = blockDim.y;
+  const bool on = !GATED || c < d;
+  const int nw = GATED ? (int)(blockDim.x >> 5) : 1, wi = GATED ? (int)(threadIdx.x >> 5) : 0;
   for (int64_t i = (int64_t)blockIdx.x * RY + ry; i < g.N; i += (int64_t)gridDim.x * RY) {
     const int kb = g.dst_ptr[i], ke = g.dst_ptr[i + 1];
     float4 num = f4zero(), den = f4zero();
-    for (int k = kb; k < ke; ++k) {
-      const int j = g.dst_src[k];
-      const int64_t eid = g.dst_eid[k];
-      const float4 s = sigmoid4(ld4(ehat + eid * d + c));
-      num = f4fma(s, ld4(Bx + (int64_t)j * ldy + c), num);
-      den = f4add(den, s);
+    if (on) {
+      for (int k = kb; k < ke; ++k) {
+        const int j = g.dst_src[k];
+        const int64_t eid = g.dst_eid[k];
+        float4 s = sigmoid4(ld4(ehat + eid * d + c));
+        if (GATED) s = f4scale(s, gate[eid]);
+        num = f4fma(s, ld4(Bx + (int64_t)j * ldy + c), num);
+        den = f4add(den, s);
+      }
     }
     const float4 inv = make_float4(1.f / (den.x + 1e-6f), 1.f / (den.y + 1e-6f), 1.f / (den.z + 1e-6f),
                                    1.f / (den.w + 1e-6f));
     const float4 agg = f4mul(num, inv);
-    const float4 gx = ld4(g_xt + i * ldg + c);
+    const float4 gx = on ? ld4(g_xt + i * ldg + c) : f4zero();
     const float4 gn = f4mul(gx, inv);                       // d/d num
     const float4 gd = make_float4(-gn.x * agg.x, -gn.y * agg.y, -gn.z * agg.z, -gn.w * agg.w);  // d/d den
-    st4(g_num + i * d + c, gn);
+    if (on) st4(g_num + i * d + c, gn);
     float4 gdx = f4zero();
     for (int k = kb; k < ke; ++k) {
-      const int j = g.dst_src[k];
       const int64_t eid = g.dst_eid[k];
-      const float4 s = sigmoid4(ld4(ehat + eid * d + c));
-      const float4 bx = ld4(Bx + (int64_t)j * ldy + c);
-      const float4 gs = f4fma(gn, bx, gd);                  // d/d sigma
-      float4 ge = ld4(g_e + eid * d + c);
-      ge.x += gs.x * s.x * (1.f - s.x);
-      ge.y += gs.y * s.y * (1.f - s.y);
-      ge.z += gs.z * s.z * (1.f - s.z);
-      ge.w += gs.w * s.w * (1.f - s.w);
-      st4(g_e + eid * d + c, ge);
-      if (g_e_p.hi) planes_store4(g_e_p, eid, c, ge);
-      gdx = f4add(gdx, ge);
+      float gsum = 0.f;
+      if (on) {
+        const int j = g.dst_src[k];
+        const float4 s = sigmoid4(ld4(ehat + eid * d + c));
+        const float4 bx = ld4(Bx + (int64_t)j * ldy + c);
+        float4 gs = f4fma(gn, bx, gd);                      // d/d sigma
+        if (GATED) {
+          gsum = gs.x * s.x + gs.y * s.y + gs.z * s.z + gs.w * s.w;
+          gs = f4scale(gs, gate[eid]);                      // d/d sigmoid(ehat)
+        }
+        float4 ge = ld4(g_e + eid * d + c);
+        ge.x += gs.x * s.x * (1.f - s.x);
+        ge.y += gs.y * s.y * (1.f - s.y);
+        ge.z += gs.z * s.z * (1.f - s.z);
+        ge.w += gs.w * s.w * (1.f - s.w);
+        st4(g_e + eid * d + c, ge);
+        if (g_e_p.hi) planes_store4(g_e_p, eid, c, ge);
+        gdx = f4add(gdx, ge);
+      }
+      if (GATED) {
+        gsum = warp_sum(gsum);
+        if ((threadIdx.x & 31) == 0) g_gate[eid * nw + wi] = gsum;
+      }
     }
-    st4(g_Dx + i * ldg + c, gdx);
-    if (g_Dx_p.hi) planes_store4(g_Dx_p, i, c, gdx);
+    if (on) {
+      st4(g_Dx + i * ldg + c, gdx);
+      if (g_Dx_p.hi) planes_store4(g_Dx_p, i, c, gdx);
+    }
   }
 }
 
+template <bool GATED>
 __global__ void k_gatedgcn_bwd_src(GpsGraph g, int d, const float* __restrict__ g_e,
                                    const float* __restrict__ ehat, const float* __restrict__ g_num,
                                    float* __restrict__ g_Ex, float* __restrict__ g_Bx, int64_t ldg, Planes g_Ex_p,
-                                   Planes g_Bx_p) {
+                                   Planes g_Bx_p, const float* __restrict__ gate) {
   const int c = threadIdx.x * 4, ry = threadIdx.y, RY = blockDim.y;
   for (int64_t j = (int64_t)blockIdx.x * RY + ry; j < g.N; j += (int64_t)gridDim.x * RY) {
     float4 gex = f4zero(), gbx = f4zero();
@@ -187,7 +219,8 @@ __global__ void k_gatedgcn_bwd_src(GpsGraph g, int d, const float* __restrict__ 
       const int i = g.src_dst[k];
       const int64_t eid = g.src_eid[k];
       gex = f4add(gex, ld4(g_e + eid * d + c));
-      const float4 s = sigmoid4(ld4(ehat + eid * d + c));
+      float4 s = sigmoid4(ld4(ehat + eid * d + c));
+      if (GATED) s = f4scale(s, gate[eid]);
       gbx = f4fma(ld4(g_num + (int64_t)i * d + c), s, gbx);
     }
     st4(g_Ex + j * ldg + c, gex);
@@ -338,36 +371,63 @@ int gcn_bwd(const GpsGraph& g, int64_t d, const float* g_h, const float* dinv, f
 }
 
 int gatedgcn_fwd(const GpsGraph& g, int64_t d, const float* Ax, const float* Bx, const float* Dx, const float* Ex,
-                 int64_t ldy, float* Ce, float* xt, double* stats_x, double* stats_e, cudaStream_t stream) {
+                 int64_t ldy, float* Ce, float* xt, double* stats_x, double* stats_e, cudaStream_t stream,
+                 const float* gate) {
   if (g.N == 0) return GPS_OK;
   NodeGeom ng;
   const bool stats = stats_x || stats_e;
   GPS_TRY(node_geom(g.N, d, stats ? 4 : 0, &ng));
-  if (stats)
-    k_gatedgcn_fwd<true><<<ng.grid, ng.block, ng.smem, stream>>>(g, (int)d, Ax, Bx, Dx, Ex, ldy, Ce, xt, stats_x,
-                                                                   stats_e);
+  if (stats && gate)
+    k_gatedgcn_fwd<true, true><<<ng.grid, ng.block, ng.smem, stream>>>(g, (int)d, Ax, Bx, Dx, Ex, ldy, Ce, xt, stats_x,
+                                                                         stats_e, gate);
+  else if (stats)
+    k_gatedgcn_fwd<true, false><<<ng.grid, ng.block, ng.smem, stream>>>(g, (int)d, Ax, Bx, Dx, Ex, ldy, Ce, xt, stats_x,
+                                                                          stats_e, nullptr);
+  else if (gate)
+    k_gatedgcn_fwd<false, true><<<ng.grid, ng.block, 0, stream>>>(g, (int)d, Ax, Bx, Dx, Ex, ldy, Ce, xt, nullptr,
+                                                                    nullptr, gate);
   else
-    k_gatedgcn_fwd<false><<<ng.grid, ng.block, 0, stream>>>(g, (int)d, Ax, Bx, Dx, Ex, ldy, Ce, xt, nullptr, nullptr);
+    k_gatedgcn_fwd<false, false><<<ng.grid, ng.block, 0, stream>>>(g, (int)d, Ax, Bx, Dx, Ex, ldy, Ce, xt, nullptr,
+                                                                     nullptr, nullptr);
   GPS_LAUNCH_CHECK();
   return GPS_OK;
 }
 
+int gatedgcn_es_nwarps(int64_t d) { return (int)(round_up(d / 4, 32) / 32); }
+
 int gatedgcn_bwd_dst(const GpsGraph& g, int64_t d, const float* g_xt, int64_t ldg, const float* ehat, const float* Bx,
-                     int64_t ldy, float* g_e, float* g_num, float* g_Dx, cudaStream_t stream, Planes g_e_p, Planes g_Dx_p) {
+                     int64_t ldy, float* g_e, float* g_num, float* g_Dx, cudaStream_t stream, Planes g_e_p, Planes g_Dx_p,
+                     const float* gate, float* g_gate) {
   if (g.N == 0) return GPS_OK;
   NodeGeom ng;
   GPS_TRY(node_geom(g.N, d, 0, &ng));
-  k_gatedgcn_bwd_dst<<<ng.grid, ng.block, 0, stream>>>(g, (int)d, g_xt, ldg, ehat, Bx, ldy, g_e, g_num, g_Dx, g_e_p, g_Dx_p);
+  if (gate) {
+    GPS_REQUIRE(g_gate, GPS_ERR_ARG, "gatedgcn_bwd_dst: the gated pass needs the g_gate buffer");
+    const int C4p = (int)round_up(d / 4, 32);   // whole warps per node row (node_geom allows d / 4 <= 1024)
+    const int RY = C4p >= 256 ? 1 : 256 / C4p;
+    const int64_t blocks = std::min<int64_t>(ceil_div(g.N, (int64_t)RY * 2), kNumSMs * 16);
+    k_gatedgcn_bwd_dst<true><<<dim3((unsigned)blocks), dim3(C4p, RY), 0, stream>>>(g, (int)d, g_xt, ldg, ehat, Bx, ldy, g_e,
+                                                                                   g_num, g_Dx, g_e_p, g_Dx_p, gate, g_gate);
+  } else {
+    k_gatedgcn_bwd_dst<false><<<ng.grid, ng.block, 0, stream>>>(g, (int)d, g_xt, ldg, ehat, Bx, ldy, g_e, g_num, g_Dx, g_e_p,
+                                                                g_Dx_p, nullptr, nullptr);
+  }
   GPS_LAUNCH_CHECK();
   return GPS_OK;
 }
 
 int gatedgcn_bwd_src(const GpsGraph& g, int64_t d, const float* g_e, const float* ehat, const float* g_num,
-                     float* g_Ex, float* g_Bx, int64_t ldg, cudaStream_t stream, Planes g_Ex_p, Planes g_Bx_p) {
+                     float* g_Ex, float* g_Bx, int64_t ldg, cudaStream_t stream, Planes g_Ex_p, Planes g_Bx_p,
+                     const float* gate) {
   if (g.N == 0) return GPS_OK;
   NodeGeom ng;
   GPS_TRY(node_geom(g.N, d, 0, &ng));
-  k_gatedgcn_bwd_src<<<ng.grid, ng.block, 0, stream>>>(g, (int)d, g_e, ehat, g_num, g_Ex, g_Bx, ldg, g_Ex_p, g_Bx_p);
+  if (gate)
+    k_gatedgcn_bwd_src<true><<<ng.grid, ng.block, 0, stream>>>(g, (int)d, g_e, ehat, g_num, g_Ex, g_Bx, ldg, g_Ex_p, g_Bx_p,
+                                                               gate);
+  else
+    k_gatedgcn_bwd_src<false><<<ng.grid, ng.block, 0, stream>>>(g, (int)d, g_e, ehat, g_num, g_Ex, g_Bx, ldg, g_Ex_p,
+                                                                g_Bx_p, nullptr);
   GPS_LAUNCH_CHECK();
   return GPS_OK;
 }

@@ -83,15 +83,18 @@ def _batch_planes_put(batch, produced, lo):
 
 
 class _GatedGCNParams(nn.Module):
-    """Parameter container with the names of graphgps/layer/gatedgcn_layer.py:21-38."""
+    """Parameter container with the names of graphgps/layer/gatedgcn_layer.py:21-38; with equivstable_pe the
+    EquivStableLapPE gate MLP `mlp_r_ij` (Linear(1,d), act, Linear(d,1), Sigmoid) sits between E and bn_node_x."""
 
-    def __init__(self, dim):
+    def __init__(self, dim, act="relu", equivstable_pe=False):
         super().__init__()
         self.A = nn.Linear(dim, dim, bias=True)
         self.B = nn.Linear(dim, dim, bias=True)
         self.C = nn.Linear(dim, dim, bias=True)
         self.D = nn.Linear(dim, dim, bias=True)
         self.E = nn.Linear(dim, dim, bias=True)
+        if equivstable_pe:
+            self.mlp_r_ij = nn.Sequential(nn.Linear(1, dim), _ACT_MODULES[act](), nn.Linear(dim, 1), nn.Sigmoid())
         self.bn_node_x = nn.BatchNorm1d(dim)
         self.bn_edge_e = nn.BatchNorm1d(dim)
 
@@ -167,7 +170,7 @@ class _GPSLayerFn(torch.autograd.Function):
     """One autograd node for the whole layer: forward = gps_layer_forward, backward = gps_layer_backward."""
 
     @staticmethod
-    def forward(ctx, layer, gs, x, e, *params):
+    def forward(ctx, layer, gs, x, e, pe, *params):
         lib = _lib.load()
         dev = x.device
         named = dict(zip(layer._param_names, params))
@@ -182,6 +185,8 @@ class _GPSLayerFn(torch.autograd.Function):
         args.x_out, args.edge_out = x_out.data_ptr(), _lib.ptr(e_out)
         args.saved, args.saved_bytes = saved.data_ptr(), saved.numel()
         args.workspace, args.workspace_bytes = ws.data_ptr(), ws.numel()
+        if layer._es:
+            args.pe, args.pe_dim = pe.data_ptr(), pe.shape[1]
         hand = layer._handoff_args(args, plan, params, x, e, x_out, e_out)
         snap = None
         if layer.training and (layer.dropout > 0 or layer.attn_dropout > 0):
@@ -192,7 +197,7 @@ class _GPSLayerFn(torch.autograd.Function):
         ctx.layer, ctx.gs, ctx.saved_buf, ctx.snap = layer, gs, saved, snap
         ctx.hand = hand
         ctx.seed, ctx.offset, ctx.training = args.seed, args.offset, bool(args.training)
-        ctx.save_for_backward(x, e, *params)
+        ctx.save_for_backward(x, e, pe, *params)
         if e_out is not None:
             return x_out, e_out
         return x_out
@@ -201,7 +206,7 @@ class _GPSLayerFn(torch.autograd.Function):
     def backward(ctx, g_x_out, g_e_out=None):
         lib = _lib.load()
         layer, gs = ctx.layer, ctx.gs
-        x, e, *params = ctx.saved_tensors
+        x, e, pe, *params = ctx.saved_tensors
         dev = x.device
         named = dict(zip(layer._param_names, params))
         bucket = layer._bucket_grads(named)
@@ -234,6 +239,12 @@ class _GPSLayerFn(torch.autograd.Function):
         args.grad_x, args.grad_edge_attr = g_x.data_ptr(), _lib.ptr(g_e)
         args.saved, args.saved_bytes = ctx.saved_buf.data_ptr(), ctx.saved_buf.numel()
         args.workspace, args.workspace_bytes = ws.data_ptr(), ws.numel()
+        g_pe = None
+        if layer._es:
+            args.pe, args.pe_dim = pe.data_ptr(), pe.shape[1]
+            if ctx.needs_input_grad[4]:
+                g_pe = torch.empty_like(pe)
+                args.grad_pe = g_pe.data_ptr()
         if ctx.hand is not None:
             args.x_planes_in, args.e_planes_in, args.wplanes, args.wplanes_bytes = ctx.hand[:4]
             args.wplanes_valid = 1
@@ -244,7 +255,7 @@ class _GPSLayerFn(torch.autograd.Function):
         _lib.check(lib.gps_layer_backward(C.byref(args), stream), "gps_layer_backward")
         # (ctx.saved_buf stays alive with the autograd node: backward(retain_graph=True) may run again)
         if bucket is not None:
-            return (None, None, g_x, g_e) + (None,) * len(layer._param_names)
+            return (None, None, g_x, g_e, g_pe) + (None,) * len(layer._param_names)
         # parameters the configuration never reads get no gradient (as under autograd in the reference)
         unused = []
         if layer.local_gnn_type == "None":
@@ -252,7 +263,7 @@ class _GPSLayerFn(torch.autograd.Function):
         if layer.global_model_type == "None":
             unused.append("norm1_attn.")
         pg = tuple(None if any(n.startswith(u) for u in unused) else grads[n] for n in layer._param_names)
-        return (None, None, g_x, g_e) + pg
+        return (None, None, g_x, g_e, g_pe) + pg
 
 
 class GPSLayer(nn.Module):
@@ -290,8 +301,13 @@ class GPSLayer(nn.Module):
         if local_gnn_type not in _SUPPORTED_LOCAL:
             raise NotImplementedError(f"local GNN '{local_gnn_type}' is not built in graphgps_b200 "
                                       f"(available: {_SUPPORTED_LOCAL}); there is no fallback path")
-        if equivstable_pe:
-            raise NotImplementedError("equivstable_pe is not built in graphgps_b200")
+        # EquivStableLapPE (gps_layer.py:66-69, 92-96, 163-171): GatedGCN gates its messages with it; GCN and None never
+        # read it (as in the reference).  The reference's GINEConvESLapPE cannot be constructed (its reset_parameters()
+        # reads mlp_r_ij before assigning it, gine_conv_layer.py:35,44,54), so there is no behaviour to reproduce.
+        if equivstable_pe and local_gnn_type == "GINE":
+            raise NotImplementedError("equivstable_pe with GINE is not built in graphgps_b200: the reference's "
+                                      "GINEConvESLapPE raises AttributeError in its own constructor")
+        self._es = bool(equivstable_pe) and local_gnn_type == "CustomGatedGCN"
         if local_gnn_type == "None":
             self.local_model = None
         elif local_gnn_type == "GINE":
@@ -300,7 +316,7 @@ class GPSLayer(nn.Module):
             self.local_gnn_with_edge_attr = False
             self.local_model = _GCNConvParams(dim_h)
         else:
-            self.local_model = _GatedGCNParams(dim_h)
+            self.local_model = _GatedGCNParams(dim_h, act, self._es)
         self.local_gnn_type = local_gnn_type
 
         # ---- global attention model (gps_layer.py:101-122)
@@ -474,6 +490,9 @@ class GPSLayer(nn.Module):
             a.gcn_D, a.gcn_E = lin("local_model.D"), lin("local_model.E")
             a.bn_node_x = bn("local_model.bn_node_x", self.local_model.bn_node_x)
             a.bn_edge_e = bn("local_model.bn_edge_e", self.local_model.bn_edge_e)
+            if self._es:
+                a.reserved1 |= _lib.ES_FLAG
+                a.es_r0, a.es_r1 = lin("local_model.mlp_r_ij.0"), lin("local_model.mlp_r_ij.2")
         elif self.local_gnn_type == "GINE":
             a.gine_lin0, a.gine_lin1 = lin("local_model.nn.0"), lin("local_model.nn.2")
             a.gine_eps = float(self._gine_eps_host)
@@ -522,11 +541,12 @@ class GPSLayer(nn.Module):
             e = e.contiguous()
         else:
             e = None
+        pe = self._pe_of(batch, x) if self._es else x.new_empty(0)
         gs = graph_of(batch)
         params = [p for _, p in self.named_parameters()]
         e_arg = e if e is not None else x.new_empty(0)
         self.__dict__["_planes_in"] = _batch_planes_get(batch)
-        out = _GPSLayerFn.apply(self, gs, x, e_arg, *params)
+        out = _GPSLayerFn.apply(self, gs, x, e_arg, pe, *params)
         produced = self.__dict__.pop("_planes_out", None)
         if self.local_gnn_type == "CustomGatedGCN":
             batch.x, batch.edge_attr = out           # gps_layer.py:173-174, :231
@@ -535,7 +555,21 @@ class GPSLayer(nn.Module):
         _batch_planes_put(batch, produced, self.precision == "fp32")
         return batch
 
+    @staticmethod
+    def _pe_of(batch, x):
+        """batch.pe_EquivStableLapPE (a missing attribute raises, as in the reference: gps_layer.py:166): [N, k] float32,
+        contiguous, on the device of batch.x.  Its gradient flows back to the PE encoder."""
+        pe = batch.pe_EquivStableLapPE
+        if not torch.is_tensor(pe) or pe.dtype != torch.float32 or pe.device != x.device:
+            raise TypeError("batch.pe_EquivStableLapPE must be a float32 tensor on the device of batch.x")
+        if pe.dim() != 2 or pe.shape[0] != x.shape[0] or pe.shape[1] == 0:
+            raise ValueError(f"batch.pe_EquivStableLapPE must be [N={x.shape[0]}, k>0] (got {tuple(pe.shape)})")
+        if not pe.is_contiguous():
+            raise ValueError("batch.pe_EquivStableLapPE must be contiguous")
+        return pe
+
     def extra_repr(self):
         return (f"summary: dim_h={self.dim_h}, local_gnn_type={self.local_gnn_type}, "
                 f"global_model_type={self.global_model_type}, heads={self.num_heads}, "
+                f"{'equivstable_pe=True, ' if self._es else ''}"
                 f"backend=libgps_b200(sm_100a), precision={self.precision}")

@@ -42,6 +42,9 @@ def register(name="gpslayer_b200"):
 
         def __init__(self, layer_config, **kwargs):
             local, glob = cfg.gt.layer_type.split("+")
+            # gps_model.py:92: equivstable_pe=cfg.posenc_EquivStableLapPE.enable (absent section: off)
+            es = getattr(getattr(cfg, "posenc_EquivStableLapPE", None), "enable", False)
+            kwargs.setdefault("equivstable_pe", bool(es))
             super().__init__(dim_h=layer_config.dim_out, local_gnn_type=local, global_model_type=glob,
                              num_heads=cfg.gt.n_heads, act=cfg.gnn.act, dropout=cfg.gt.dropout,
                              attn_dropout=cfg.gt.attn_dropout, layer_norm=cfg.gt.layer_norm,

@@ -52,22 +52,28 @@ class GPSStack(nn.Module):
         """Records `bucket.zero_(); out = stack(batch); backward(out, cotangents); collective()` into one CUDA graph.
 
         `batch` must be resident on the GPU with its graph structure already built (graph.graph_of); its x / edge_attr
-        are the graph's static inputs (copy new data into them before replay()).  Returns a CapturedStep."""
+        (and pe_EquivStableLapPE when present, for equivstable_pe layers) are the graph's static inputs (copy new data
+        into them before replay()).  Returns a CapturedStep."""
         from .batch import GraphBatch
         from .graph import graph_of
         gs = graph_of(batch)
         x_in = batch.x.detach().requires_grad_(True)
         e_in = batch.edge_attr.detach().requires_grad_(True) if getattr(batch, "edge_attr", None) is not None else None
+        pe = getattr(batch, "pe_EquivStableLapPE", None)
+        pe_in = pe.detach().requires_grad_(True) if pe is not None else None
+        extra = {"pe_EquivStableLapPE": pe_in} if pe_in is not None else {}
         params = [p for p in self.parameters()]
         res = {}
 
         def body():
             bb = GraphBatch(x=x_in, edge_index=batch.edge_index, edge_attr=e_in, batch=batch.batch,
-                            num_graphs=batch.num_graphs)
+                            num_graphs=batch.num_graphs, **extra)
             bb.__dict__["_gps_b200_graph"] = gs
             x_in.grad = None
             if e_in is not None:
                 e_in.grad = None
+            if pe_in is not None:
+                pe_in.grad = None
             if bucket is not None:
                 bucket.zero_()
             else:
@@ -93,14 +99,15 @@ class GPSStack(nn.Module):
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, capture_error_mode="thread_local"):
             body()
-        return CapturedStep(g, x_in, e_in, res["x"], res["e"])
+        return CapturedStep(g, x_in, e_in, res["x"], res["e"], pe_in)
 
 
 class CapturedStep:
     """One captured forward+backward of a GPSStack: static inputs, outputs and input gradients."""
 
-    def __init__(self, graph, x_in, e_in, x_out, e_out):
+    def __init__(self, graph, x_in, e_in, x_out, e_out, pe_in=None):
         self.graph, self.x_in, self.e_in, self.x_out, self.e_out = graph, x_in, e_in, x_out, e_out
+        self.pe_in = pe_in
 
     def replay(self):
         self.graph.replay()
@@ -112,3 +119,8 @@ class CapturedStep:
     @property
     def grad_e(self):
         return self.e_in.grad if self.e_in is not None else None
+
+    @property
+    def grad_pe(self):
+        """Gradient w.r.t. the batch's pe_EquivStableLapPE summed over the layers (None without one)."""
+        return self.pe_in.grad if self.pe_in is not None else None

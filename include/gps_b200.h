@@ -136,7 +136,7 @@ typedef struct {
   uint64_t seed;             /* Philox key for this call's dropout masks            */
   uint64_t offset;           /* Philox counter base (caller advances per call)      */
   float gine_eps;            /* local_model.eps buffer value (GINE)                 */
-  int32_t reserved1;
+  int32_t reserved1;         /* flags; bit 0: EquivStableLapPE edge gate (fields pe .. es_r1 at the end)  */
 
   GpsGraph graph;
 
@@ -200,6 +200,20 @@ typedef struct {
    * backward is done, the in_proj block at the end.  ev_grads_done: every gradient of this layer is final. */
   void* ev_grads_mid;
   void* ev_grads_done;
+
+  /* EquivStableLapPE edge gate of the GatedGCN local model (GPSLayer(..., equivstable_pe=True): gatedgcn_layer.py:29-35,
+   * 63-70, 99-103), switched on by reserved1 bit 0 and read ONLY then, so a zero-initialised caller never reaches these
+   * fields.  With the bit set for a local model other than GatedGCN the calls return GPS_ERR_UNSUPPORTED.
+   *   r_ij = sum_c (pe_i,c - pe_j,c)^2,  gate_ij = sigmoid(W2 act(W1 r_ij + b1) + b2),  sigma_ij = sigmoid(e_ij) * gate_ij
+   * in the aggregation (the edge output e_ij stays ungated).  fp32 in both precision modes.
+   *   pe       batch.pe_EquivStableLapPE [N, pe_dim], row-major float32 (the same tensor for every layer);
+   *   grad_pe  backward output [N, pe_dim], overwritten (not accumulated); NULL = not computed;
+   *   es_r0    local_model.mlp_r_ij.0 (weight [d,1], bias [d]);  es_r1  local_model.mlp_r_ij.2 (weight [1,d], bias [1]).
+   * Their gradients follow reserved0 like every other parameter and belong to the ev_grads_mid group. */
+  const float* pe;
+  int64_t pe_dim;
+  float* grad_pe;
+  GpsLinear es_r0, es_r1;
 } GpsLayerArgs;
 
 typedef struct {
@@ -244,6 +258,27 @@ int gps_gemm(const float* A, int64_t lda, int32_t ta, const float* B, int64_t ld
 int gps_gatedgcn_aggregate_forward(const GpsGraph* g, int64_t d, const float* Ax, const float* Bx,
                                    const float* Dx, const float* Ex, int64_t ldy, float* Ce,
                                    float* xt, double* stats_x, double* stats_e, void* stream);
+
+/* EquivStableLapPE edge gate (see GpsLayerArgs.pe): r [E] and gate [E] per original edge id.  w0/b0 = mlp_r_ij.0,
+ * w2/b2 = mlp_r_ij.2, act = GPS_ACT_*. */
+int gps_es_gate_forward(const GpsGraph* g, const float* pe, int64_t pe_dim, int64_t d, int32_t act,
+                        const float* w0, const float* b0, const float* w2, const float* b2, float* r, float* gate,
+                        void* stream);
+/* gps_gatedgcn_aggregate_forward with sigma_ij = sigmoid(e_ij) * gate[edge id]. */
+int gps_gatedgcn_es_aggregate_forward(const GpsGraph* g, int64_t d, const float* Ax, const float* Bx,
+                                      const float* Dx, const float* Ex, int64_t ldy, float* Ce, float* xt,
+                                      double* stats_x, double* stats_e, const float* gate, void* stream);
+/* Backward of the gate MLP: given g_gate [E] = d loss / d gate, writes g_r [E] = d loss / d r and the four
+ * mlp_r_ij gradients (overwritten).  Deterministic (per-block partials in `workspace`, fixed-order final sum);
+ * workspace_bytes >= gps_es_gate_backward_workspace_bytes(E, d). */
+int64_t gps_es_gate_backward_workspace_bytes(int64_t E, int64_t d);
+int gps_es_gate_backward(int64_t E, int64_t d, int32_t act, const float* w0, const float* b0, const float* w2,
+                         const float* b2, const float* r, const float* gate, const float* g_gate, float* g_r,
+                         float* grad_w0, float* grad_b0, float* grad_w2, float* grad_b2, void* workspace,
+                         int64_t workspace_bytes, void* stream);
+/* d loss / d pe from g_r: grad_pe_n = sum_{e: dst=n} 2 g_r_e (pe_n - pe_src(e)) + sum_{e: src=n} 2 g_r_e (pe_n - pe_dst(e)) */
+int gps_es_pe_backward(const GpsGraph* g, const float* pe, int64_t pe_dim, const float* g_r, float* grad_pe,
+                       void* stream);
 
 /* GINE aggregate: out_i = (1+eps)·x_i + Σ_{j→i} relu(x_j + e_ij)  (gine_conv_layer.py:56-84) */
 int gps_gine_aggregate_forward(const GpsGraph* g, int64_t d, const float* x, const float* e,
